@@ -1,6 +1,7 @@
 """bench.py — DSA inputs prioritized / second on B200 (BASELINE.json metric), driver contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c1|c2|c3|c4|c5s]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic test traces.
@@ -402,6 +403,29 @@ def run_c5_slice(args, tm: Timer, dev, rank, world, comm, steps: int, cfg=None):
 # ----------------------------------------------------------------------------------------------
 # our arm: C2 headline
 # ----------------------------------------------------------------------------------------------
+def step_outputs(out, plan, order, x_sorted, x_raw):
+    """What one C2 device step computed, as a DSA caller receives it: float64 arrays with one entry per test input,
+    in the order of the test inputs.  `out` is the step's result: the plan's [4, n] buffer, whose column r belongs to
+    row r of the plan's landing buffer (class-sorted after load_sorted, the caller's rows after a DSA call), or, for
+    an eager step, dist_a / dist_b of the class-sorted rows."""
+    import torch
+
+    if plan is None:
+        named, rows = {"dsa": out}, order
+    else:
+        named = dict(zip(("dist_a", "dist_b", "winner_index", "dsa"), out))
+        if torch.equal(plan.x_in, x_sorted):
+            rows = order
+        else:
+            assert torch.equal(plan.x_in, x_raw), "the plan's landing buffer holds neither row order of the test inputs"
+            rows = np.arange(order.size)
+    res = {}
+    for name, v in named.items():
+        res[name] = np.empty(order.size)
+        res[name][rows] = v.double().cpu().numpy()
+    return res
+
+
 def run_ours(args):
     import torch
 
@@ -478,10 +502,11 @@ def run_ours(args):
         a, b, _ = E.dsa_distances(eng, x_sorted, q_class, q_off, main_comm)
         return a / b
 
+    last = {}
+
     def step_device():
-        if plan is None:
-            return step_eager()
-        return plan.run()[3]
+        # keeps the step's result referenced: --dump-outputs reads what the last timed step computed
+        last["out"] = step_eager() if plan is None else plan.run()
 
     def step_e2e():
         return sa(xte_host, pte)
@@ -514,6 +539,7 @@ def run_ours(args):
     if plan is not None and plan.speculative:
         # the replayed graph carries no exhaustive-scan launches; it is only valid if no candidate list overflowed
         assert int(plan.overflow.item()) == 0, "a candidate list overflowed: the timed graph did not produce the result"
+    dumped = step_outputs(last["out"], plan, order, x_sorted, xte_dev) if (args.dump_outputs and rank == 0) else None
     t_e2e = tm.timed(step_e2e, args.steps)
     t_page = tm.timed(step_e2e_pageable, args.steps)
     step_api_device()
@@ -590,7 +616,7 @@ def run_ours(args):
         sa._engine._plans.clear()
         torch.cuda.empty_cache()
         try:
-            c5 = run_c5_slice(args, tm, dev, rank, world, comm, steps=min(args.steps, 10))
+            c5 = run_c5_slice(args, tm, dev, rank, world, comm, steps=args.steps)
         except Exception as e:   # pragma: no cover - keep the headline line even if the big slice fails
             import traceback
 
@@ -603,7 +629,7 @@ def run_ours(args):
         others = {}
         for wl in ("c1", "c3", "c4", "cam"):
             try:
-                others[wl] = secondary(wl, args, tm, dev, steps=min(args.steps, 10), with_cpu=not args.no_cpu)
+                others[wl] = secondary(wl, args, tm, dev, steps=args.steps, with_cpu=not args.no_cpu)
             except Exception as e:   # pragma: no cover
                 others[wl] = {"error": f"{type(e).__name__}: {e}"}
 
@@ -674,6 +700,10 @@ def run_ours(args):
             line["other_configs"] = others
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_baseline(xtr, ytr, xte, pte)
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, v in dumped.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), v)
         sys.stdout.flush()
         os.dup2(saved_stdout, 1)
         print(json.dumps(line), flush=True)
@@ -959,7 +989,7 @@ def run_secondary(args):
     sampler = ClockSampler(0)
     sampler.start()
     if args.workload == "c5s":
-        line = run_c5_slice(args, tm, dev, 0, 1, None, steps=min(args.steps, 10))
+        line = run_c5_slice(args, tm, dev, 0, 1, None, steps=args.steps)
     else:
         line = secondary(args.workload, args, tm, dev, args.steps, with_cpu=not args.no_cpu)
     line["clocks"] = sampler.stop()
@@ -986,7 +1016,14 @@ def main():
     ap.add_argument("--workload", default="c2", choices=["c1", "c2", "c3", "c4", "c5s", "cam"],
                     help="c2 (default) = the configuration the headline metric is quoted on (its line also carries the "
                          "others); c1/c3/c4/c5s = one of the other configurations alone, single GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed C2 step computed as DIR/<name>.npy: dsa, "
+                         "dist_a, dist_b, winner_index, float64, one entry per test input (rank 0's), in input order")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the outputs of the C2 headline (--impl ours --workload c2)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload != "c2":
