@@ -222,8 +222,7 @@ int tip_nn_filter(const void* q_pack, const float* q_sqnorm, int64_t m, const vo
  * is the train-tile height (256 or 128), useful for sizing spans. */
 int tip_nn_filter_tile(int64_t d, int32_t* q_rows, int32_t* t_rows);
 /* which tensor-core kernel tip_nn_filter runs for traces of width d: 1 = resident-query (d <= 128, 256 x 192
- * tiles), 2 = streaming CTA pair (cta_group::2, 256 x 256 tiles per pair of SMs), 0 = streaming single CTA
- * (128 x 256 tiles; B200TIP_PAIR2=0).  tip_kde_tile_rows: query rows per work item of tip_kde_lse*. */
+ * tiles), 0 = streaming (128 x 256 tiles).  tip_kde_tile_rows: query rows per work item of tip_kde_lse*. */
 int tip_nn_filter_kind(int64_t d);
 int tip_kde_tile_rows(void);
 int tip_kde_slot_parts(void);   /* partial (max, sum) pairs per work-item slot: part_max / part_sum hold slots x this x m */
@@ -384,8 +383,7 @@ int tip_kde_combine(const float* part_max, const float* part_sum, int64_t m, int
 /* ---- bring-up / validation: plain accumulator dump ------------------------------------
  * out[256*256] (fp32, row-major, leading dimension 256) = tail-augmented dot products of q rows
  * [0,128) (streaming kernel) or [0,256) (resident-query kernel) with t rows [0,256).
- * variant: 0 = the kernel tip_nn_filter would pick, 1 = streaming, 2 = resident-query, 3 = streaming CTA pair
- * (q rows [0,256)). */
+ * variant: 0 = the kernel tip_nn_filter would pick, 1 = streaming, 2 = resident-query. */
 int tip_pair_probe(const void* q_pack, int64_t m, const void* t_pack, int64_t n, int64_t d,
                    int segments, int64_t pitch, int variant, float* out, void* stream);
 

@@ -39,18 +39,6 @@ void count_launch(int n = 1);
 
 int sm_count();
 
-// The kernels that run between two launches of the tcgen05 filter inside one scoring call ask for the same
-// shared-memory carve-out as the filter (max shared), so that the SMs are not re-partitioned at every kernel
-// boundary of the chain.  B200TIP_CARVEOUT=0 leaves the driver's default (A/B knob).
-bool carveout_enabled();
-template <typename K>
-inline void prefer_max_shared(K kernel, bool* done) {
-  if (*done) return;
-  *done = true;
-  if (carveout_enabled())
-    (void)cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-}
-
 // ---- IEEE arithmetic without FMA contraction (NumPy never fuses) --------------------------
 template <typename T> struct Rn;
 template <> struct Rn<float> {
@@ -336,16 +324,14 @@ __device__ __forceinline__ uint32_t seed_row_min_bits(float ub, float nx, float 
 // One query row -> packed bf16 operand of tip_nn_filter (one segment) + reset filter state, by a full
 // warp: the arithmetic of pair_prep_kernel (query role): centre in fp32, round to bf16, |h|^2 and
 // the dropped part's norm accumulated in double.  src == nullptr packs a zero row.
-template <typename T, int NL = 32>
+template <typename T>
 __device__ __forceinline__ void warp_pack_query(const T* __restrict__ src, int d, const float* __restrict__ center,
                                                 __nv_bfloat16* __restrict__ out, int64_t pitch, float* sqnorm,
                                                 float* rounderr, uint32_t* row_min, int32_t* cand_cnt, int lane,
-                                                float seed_ub = 3.4e38f, const SeedParams* sp = nullptr,
-                                                unsigned mask = 0xffffffffu) {
-  // NL cooperating lanes (a full warp, or one 8-lane group of it: `lane` in [0, NL), `mask` names the group)
+                                                float seed_ub = 3.4e38f, const SeedParams* sp = nullptr) {
   const int d16 = (d + 15) & ~15;
   double acc = 0.0, err = 0.0;
-  for (int c = lane; c < d16; c += NL) {
+  for (int c = lane; c < d16; c += 32) {
     float v = 0.f;
     if (c < d) {
       const T xv = src ? src[c] : (T)0;
@@ -360,11 +346,11 @@ __device__ __forceinline__ void warp_pack_query(const T* __restrict__ src, int d
     out[c] = h;
   }
 #pragma unroll
-  for (int o = NL / 2; o > 0; o >>= 1) {
-    acc += __shfl_xor_sync(mask, acc, o);
-    err += __shfl_xor_sync(mask, err, o);
+  for (int o = 16; o > 0; o >>= 1) {
+    acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    err += __shfl_xor_sync(0xffffffffu, err, o);
   }
-  for (int c = d16 + lane; c < pitch; c += NL) out[c] = __float2bfloat16_rn(c - d16 < 3 ? 1.f : 0.f);
+  for (int c = d16 + lane; c < pitch; c += 32) out[c] = __float2bfloat16_rn(c - d16 < 3 ? 1.f : 0.f);
   if (lane == 0) {
     const float nx = (float)acc;
     const float qe = (float)sqrt(err) * 1.000001f;

@@ -19,7 +19,6 @@
 #include <cudaTypedefs.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace tip {
@@ -33,7 +32,6 @@ constexpr int kBBytes = BN * BK * 2;
 constexpr int kStageBytes = kABytes + kBBytes;
 constexpr int kResAChunks = 5;               // resident-A variant (RESA): query tiles of up to 5 x 64 K elements
 constexpr int kEpiThreads = 256;             // 8 epilogue warps
-constexpr int kThreads = 64 + kEpiThreads;   // + TMA warp + MMA warp
 // epilogue warps of the streaming kernel in log-sum-exp mode (8 or 16, see pair_kernel).  16 was measured at C3 and
 // changes nothing (0.338 ms either way): the K = 272 pass is bound by shared-memory bandwidth — both operands stream
 // through shared memory for every tile (TMA writes 94 B/clk + MMA reads 96 B/clk against a 128 B/clk port = the
@@ -77,9 +75,6 @@ struct PairArgs {
   int timeline_tiles;
   // bring-up: per-CTA {globaltimer at start, at end, tiles, items} of the resident kernel, or nullptr
   long long* cta_clock;
-  // resident kernel: the query tile's full 64-element K chunks are copied into the free TMEM columns [192, 256) of each
-  // accumulator half once per query tile and the MMAs read A from there (the K tail stays in shared memory)
-  int a_tmem;
 };
 
 // ---- PTX wrappers --------------------------------------------------------------------------
@@ -106,10 +101,10 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   return ok != 0;
 }
 // Bounded spin: a protocol bug must surface as a trapped kernel, never as a hung GPU.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, uint32_t max_spins = 200000000u) {
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
-    if (++spins > max_spins) __trap();
+    if (++spins > 200000000u) __trap();
   }
 }
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1) {
@@ -195,54 +190,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
       : "r"(taddr));
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// ---- cta_group::2 (CTA pair) wrappers ---------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `addr` (a shared::cta address of this CTA) in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA load into THIS CTA's shared memory whose bytes are counted on a barrier of the pair's leader CTA
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, uint32_t bar_cluster, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst), "l"(map), "r"(bar_cluster), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma2_acc(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.eq.u32 p, 1, 1;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc)
-      : "memory");
-}
-__device__ __forceinline__ void umma2_first(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.eq.u32 p, 1, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc)
-      : "memory");
-}
-// arrives (once the MMAs issued so far retire) on the barrier at the same offset in BOTH CTAs of the pair
-__device__ __forceinline__ void umma2_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)3)
-               : "memory");
-}
 
 // K-major, 128-byte-swizzled operand tile: rows of 128 B, 8-row groups 1024 B apart
 // (cute::UMMA::SmemDescriptor: start>>4 | LBO=1<<16 | SBO=64<<32 | version=1<<46 | SWIZZLE_128B=2<<61).
@@ -662,248 +609,6 @@ pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 }
 
 // =============================================================================================
-// CTA-pair variant of the streaming kernel (cta_group::2): two CTAs of a cluster compute a 256 x 256 tile.
-// Each CTA owns 128 query rows (its accumulators live in its own TMEM, its epilogue warps reduce them) and
-// stages only HALF of every 256-row train chunk; the pair's leader issues M256 x N256 x K16 MMAs that read
-// A from both CTAs and the two B halves from both CTAs' shared memory.  Per CTA and K16 step the tensor
-// pipe now reads 4 KB of A + 4 KB of B (64 B/clk) and TMA writes 32 KB per 64-wide chunk (64 B/clk):
-// together the 128 B/clk a shared-memory port delivers, against 192 B/clk asked by the single-CTA
-// 128 x 256 tile, which capped that kernel at ~2/3 of the tensor peak; L2 -> SM traffic per flop drops by a
-// third as well.  Barriers: TMA bytes of both CTAs are counted on the LEADER's full barriers (the leader's
-// producer arms them with the pair's byte count, the peer's producer arrives remotely); tcgen05.commit
-// multicasts to both CTAs' empty / accumulator-full barriers; both CTAs' epilogue warps release the
-// accumulator stage on the leader's barrier.
-// =============================================================================================
-constexpr int kP2Stages = 6;
-constexpr uint32_t kP2Spins = 20000000u;   // a protocol bug traps within seconds
-constexpr int kP2ABytes = 128 * BK * 2;
-constexpr int kP2BBytes = 128 * BK * 2;
-constexpr int kP2StageBytes = kP2ABytes + kP2BBytes;
-constexpr int kP2SmemBytes = kP2Stages * kP2StageBytes + 1024 + 256 + kCandBytes;
-static_assert(kP2SmemBytes <= 232448, "pair kernel does not fit");
-constexpr uint32_t kIdescP2 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-constexpr uint32_t kIdescP2F16 = (1u << 4) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-
-template <int MODE, bool EXCL>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-pair2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const PairArgs args) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t raw = smem_u32(smem_raw);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  uint8_t* smem = smem_raw + (base - raw);
-  const uint32_t bar0 = base + kP2Stages * kP2StageBytes;
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (kP2Stages + s); };
-  auto tfull_bar = [&](int a) { return bar0 + 8u * (2 * kP2Stages + a); };
-  auto tempty_bar = [&](int a) { return bar0 + 8u * (2 * kP2Stages + 2 + a); };
-  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + kP2Stages * kP2StageBytes + 8 * (2 * kP2Stages + 4));
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader_cta = rank == 0;
-  const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
-    for (int s = 0; s < kP2Stages; s++) { mbar_init(full_bar(s), 2); mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < 2; a++) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 2 * (kEpiThreads / 32)); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)),
-                 "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const int k16 = args.k16;
-  const int nchunks = (k16 + 3) >> 2;
-
-  if (warp == 0) {
-    // ================= TMA producer (both CTAs) =================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int w = pair; w < args.n_items; w += n_pairs) {
-        const tip_work_item it = args.items[w];
-        const int ntiles = (it.col1 - it.col0 + BN - 1) / BN;
-        for (int t = 0; t < ntiles; t++) {
-          for (int c = 0; c < nchunks; c++) {
-            mbar_wait(empty_bar(stage), phase ^ 1u, kP2Spins);
-            const uint32_t lead_full = mapa_shared(full_bar(stage), 0);
-            if (leader_cta) mbar_expect_tx(full_bar(stage), 2 * kP2StageBytes);
-            const uint32_t a_dst = base + stage * kP2StageBytes;
-            tma_load_2d_pair(a_dst, &tmA, lead_full, c * BK, it.q_row0 + (int)rank * 128);
-            tma_load_2d_pair(a_dst + kP2ABytes, &tmB, lead_full, c * BK, it.col0 + t * BN + (int)rank * 128);
-            if (!leader_cta) mbar_arrive_cluster(lead_full);
-            if (++stage == kP2Stages) { stage = 0; phase ^= 1u; }
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // ================= MMA issuer (leader CTA of the pair) =================
-    if (leader_cta) {
-      const bool leader = elect_one();
-      const uint32_t idesc = args.idesc ? args.idesc : kIdescP2;
-      int stage = 0, acc = 0;
-      uint32_t phase = 0, acc_phase = 0;
-      for (int w = pair; w < args.n_items; w += n_pairs) {
-        const tip_work_item it = args.items[w];
-        const int ntiles = (it.col1 - it.col0 + BN - 1) / BN;
-        for (int t = 0; t < ntiles; t++) {
-          mbar_wait(tempty_bar(acc), acc_phase ^ 1u, kP2Spins);
-          tc_fence_after();
-          const uint32_t d_tmem = tmem_base + (uint32_t)acc * BN;
-          for (int c = 0; c < nchunks; c++) {
-            mbar_wait(full_bar(stage), phase, kP2Spins);
-            tc_fence_after();
-            const uint32_t a_addr = base + stage * kP2StageBytes;
-            const uint64_t adesc = smem_desc(a_addr);
-            const uint64_t bdesc = smem_desc(a_addr + kP2ABytes);
-            const int nm = min(4, k16 - 4 * c);
-            if (leader) {
-              // straight-line issue (a single thread's dependent stream costs ~45 cycles per instruction: no loop
-              // counters, no runtime predicates on the common path)
-              if (c == 0) umma2_first(d_tmem, adesc, bdesc, idesc);
-              else umma2_acc(d_tmem, adesc, bdesc, idesc);
-              if (nm == 4) {
-                umma2_acc(d_tmem, adesc + 2u, bdesc + 2u, idesc);
-                umma2_acc(d_tmem, adesc + 4u, bdesc + 4u, idesc);
-                umma2_acc(d_tmem, adesc + 6u, bdesc + 6u, idesc);
-              } else {
-                for (int k = 1; k < nm; k++) umma2_acc(d_tmem, adesc + 2u * k, bdesc + 2u * k, idesc);
-              }
-              umma2_commit(empty_bar(stage));
-              if (c == nchunks - 1) umma2_commit(tfull_bar(acc));
-            }
-            __syncwarp();
-            if (++stage == kP2Stages) { stage = 0; phase ^= 1u; }
-          }
-          acc ^= 1;
-          if (acc == 0) acc_phase ^= 1u;
-        }
-      }
-    }
-  } else {
-    // ================= epilogue (both CTAs: own 128 query rows x 256 columns) =================
-    const int quad = warp & 3;
-    const int half = (warp - 2) >> 2;
-    const int row_local = quad * 32 + lane;
-    const uint32_t lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(half * (BN / 2));
-    const int etid = threadIdx.x - 64;
-    EpiShared sh;
-    sh.cand_val = reinterpret_cast<float*>(smem + kP2Stages * kP2StageBytes + 256);
-    sh.cand_col = reinterpret_cast<int*>(sh.cand_val + kCandSlots * kEpiThreads);
-    sh.cand_mask = reinterpret_cast<uint32_t*>(sh.cand_col + kCandSlots * kEpiThreads);
-    sh.etid = etid;
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    const float kInf = __int_as_float(0x7f800000);
-    for (int w = pair; w < args.n_items; w += n_pairs) {
-      const tip_work_item it = args.items[w];
-      const int ntiles = (it.col1 - it.col0 + BN - 1) / BN;
-      EpiState st;
-      const int row_in_item = (int)rank * 128 + row_local;
-      st.valid_row = row_in_item < it.q_rows;
-      st.row = (int64_t)it.q_row0 + row_in_item;
-      st.nx = 0.f; st.e2 = 0.f; st.g = 0.f; st.best = kInf; st.thr = kInf; st.s_ref = kInf; st.n_staged = 0;
-      st.run_max = -kInf; st.run_sum = 0.f;
-      st.col1 = it.col1;
-      st.ex_lo = 0; st.ex_hi = 0;
-      if (MODE == MODE_NN && st.valid_row) {
-        if (EXCL && (it.reserved & 1) && args.q_class) {
-          const int cls = args.q_class[st.row];
-          st.ex_lo = args.class_off[cls];
-          st.ex_hi = args.class_off[cls + 1];
-        }
-        st.nx = args.q_sqnorm[st.row];
-        const float r = sqrtf(st.nx) + args.rmax;
-        st.e2 = args.q_err ? 2.f * (args.q_err[st.row] + args.t_err + 1.2e-7f * r) * 1.00001f : args.eps2 * r;
-        st.g = args.gamma * r * r;
-        st.s_ref = __uint_as_float(ld_volatile_u32(args.row_min_bits + st.row));
-        st.thr = nn_threshold(st.s_ref, st.nx, st.e2, st.g);
-      }
-      for (int t = 0; t < ntiles; t++) {
-        mbar_wait(tfull_bar(acc), acc_phase, kP2Spins);
-        tc_fence_after();
-        const int col_base = it.col0 + t * BN + half * (BN / 2);
-        const bool partial = col_base + BN / 2 > it.col1;
-        uint32_t seen_bits = 0x7f800000u;
-        if (MODE == MODE_NN && st.valid_row) seen_bits = ld_volatile_u32(args.row_min_bits + st.row);
-        const uint32_t taddr = lane_addr + (uint32_t)(acc * BN);
-        uint32_t ra[32], rb[32];
-        tmem_ld32(taddr, ra);
-#pragma unroll 1
-        for (int h = 0; h < 2; h++) {
-          tmem_wait_ld();
-          tmem_ld32(taddr + 64 * h + 32, rb);
-          epi_chunk<MODE, EXCL>(args, st, sh, ra, col_base + 64 * h, partial, w == 0 && t == 0, row_in_item,
-                                half * (BN / 2) + 64 * h);
-          tmem_wait_ld();
-          if (h == 0) {
-            tmem_ld32(taddr + 64, ra);
-          } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty_bar(acc), 0));
-          }
-          epi_chunk<MODE, EXCL>(args, st, sh, rb, col_base + 64 * h + 32, partial, w == 0 && t == 0, row_in_item,
-                                half * (BN / 2) + 64 * h + 32);
-        }
-        if (MODE == MODE_NN && st.valid_row) {
-          const float mine = fmaxf(st.best + st.nx, 0.f);
-          const float seen = __uint_as_float(seen_bits);
-          if (mine < seen) atomicMin(args.row_min_bits + st.row, __float_as_uint(mine));
-          if (seen < st.s_ref) {
-            st.s_ref = seen;
-            st.thr = nn_threshold(st.s_ref, st.nx, st.e2, st.g);
-          }
-        }
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1u;
-      }
-      if (MODE == MODE_NN) {
-        if (st.valid_row) {
-          const float seen = __uint_as_float(ld_volatile_u32(args.row_min_bits + st.row));
-          if (seen < st.s_ref) {
-            st.s_ref = seen;
-            st.thr = nn_threshold(st.s_ref, st.nx, st.e2, st.g);
-          }
-          for (int k = 0; k < st.n_staged; k++) {
-            if (sh.cand_val[k * kEpiThreads + etid] <= st.thr) {
-              const int pos = atomicAdd(args.cand_cnt + st.row, 1);
-              if (pos < args.cap) {
-                args.cand_idx[(st.row * args.cap + pos) * 2] = sh.cand_col[k * kEpiThreads + etid];
-                args.cand_idx[(st.row * args.cap + pos) * 2 + 1] = (int)sh.cand_mask[k * kEpiThreads + etid];
-              }
-            }
-          }
-        }
-      } else if (MODE == MODE_LSE) {
-        if (st.valid_row) {
-          args.part_max[(int64_t)(it.slot * 2 + half) * args.m + st.row] = st.run_max;
-          args.part_sum[(int64_t)(it.slot * 2 + half) * args.m + st.row] = st.run_sum;
-        }
-      }
-    }
-  }
-
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-  }
-}
-
-// =============================================================================================
 // Resident-query variant for short traces (packed width <= 9 K-steps, e.g. D = 128):
 // 256 query rows stay in shared memory for a whole work item and 192-row train tiles are
 // streamed (2-stage ring), so the L2 -> SM traffic per 256 x 192 output tile is the train tile
@@ -986,7 +691,10 @@ pair_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const uint32_t b_base = a_base + geo.a_bytes;
   const uint32_t a_rem2 = b_base + (uint32_t)kRsStages * geo.b_bytes;     // see rs_tail_bytes
   constexpr uint32_t tiles_bytes = geo.a_bytes + (uint32_t)kRsStages * geo.b_bytes + (uint32_t)rs_tail_bytes(K16);
-  const bool ta = args.a_tmem && NFULL > 0;
+  // A from tensor memory: the query tile's full 64-element K chunks are copied into the free TMEM columns [192, 256)
+  // of each accumulator half once per query tile and the MMAs read A from there (the K tail stays in shared memory;
+  // measured at C2: 0.186 -> 0.183 ms per step).  With no full chunk (d < 64) A is read from shared memory.
+  constexpr bool ta = NFULL > 0;
   const uint32_t bar0 = base + tiles_bytes;
   // barriers: 0 a_full, 1 a_empty, 2..3 b_full, 4..5 b_empty, 20..23 tfull[quarter], 24..27 tempty[quarter],
   // 10..11 sched_full[slot], 12..13 sched_empty[slot]; then the TMEM base and the 2-slot item ring
@@ -1365,7 +1073,6 @@ static int check_device() {
   return TIP_OK;
 }
 
-constexpr int kResADefault = 1;      // measured at C3: 0.3406 -> 0.3320 ms per step
 static_assert(kResAChunks * kABytes + kStages * kBBytes + 256 + 1024 <= kSmemBytes, "resident-A layout does not fit");
 
 template <int MODE, bool EXCL = false>
@@ -1390,44 +1097,14 @@ static int launch_pair(const void* q_pack, int64_t m, const void* t_pack, int64_
     attr_set = true;
   }
   const int grid = min(args.n_items, sm_count());
-  static int resa = -1;      // B200TIP_RESA=0: the log-sum-exp pass streams the query tile like the candidate search does
-  if (resa < 0) {
-    const char* e = getenv("B200TIP_RESA");
-    resa = e ? (e[0] == '1' ? 1 : 0) : kResADefault;
-  }
-  if (MODE == MODE_LSE && resa && (args.k16 + 3) / 4 <= kResAChunks)
+  // a query tile that fits stays resident in the log-sum-exp pass (measured at C3: 0.3406 -> 0.3320 ms per step)
+  if (MODE == MODE_LSE && (args.k16 + 3) / 4 <= kResAChunks)
     pair_kernel<MODE, EXCL, EW, MODE == MODE_LSE><<<grid, 64 + 32 * EW, kSmemBytes, st>>>(ma, mb, args);
   else
     pair_kernel<MODE, EXCL, EW><<<grid, 64 + 32 * EW, kSmemBytes, st>>>(ma, mb, args);
   TIP_LAUNCH_CHECK();
   return TIP_OK;
 }
-
-template <int MODE, bool EXCL = false>
-static int launch_pair2(const void* q_pack, int64_t m, const void* t_pack, int64_t n, int64_t pitch, PairArgs args,
-                        cudaStream_t st) {
-  int rc = check_device();
-  if (rc != TIP_OK) return rc;
-  TIP_REQUIRE(((uintptr_t)q_pack & 127) == 0 && ((uintptr_t)t_pack & 127) == 0, "packed operands must be 128-byte aligned");
-  TIP_REQUIRE(pitch % 64 == 0 && args.k16 * 16 <= pitch, "pitch");
-  TIP_REQUIRE(m >= 1 && n >= 1 && m < (1LL << 31) && n < (1LL << 31), "shape");
-  CUtensorMap ma, mb;
-  rc = make_map(&ma, q_pack, m, pitch, 128);
-  if (rc != TIP_OK) return rc;
-  rc = make_map(&mb, t_pack, n, pitch, 128);
-  if (rc != TIP_OK) return rc;
-  static bool attr_set = false;   // one flag per template instantiation
-  if (!attr_set) {
-    TIP_CHECK_CUDA(cudaFuncSetAttribute(pair2_kernel<MODE, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP2SmemBytes));
-    attr_set = true;
-  }
-  const int pairs = std::max(1, std::min(args.n_items, sm_count() / 2));
-  pair2_kernel<MODE, EXCL><<<2 * pairs, kThreads, kP2SmemBytes, st>>>(ma, mb, args);
-  TIP_LAUNCH_CHECK();
-  return TIP_OK;
-}
-
-constexpr int kATmemDefault = 1;   // measured at C2: stage 2 0.124-0.132 -> 0.120 ms, step 0.186 -> 0.183 ms (A/B on one box)
 
 template <int MODE, bool EXCL = false>
 static int launch_pair_rs(const void* q_pack, int64_t m, const void* t_pack, int64_t n, int64_t pitch, PairArgs args,
@@ -1459,12 +1136,6 @@ static int launch_pair_rs(const void* q_pack, int64_t m, const void* t_pack, int
   }
   const int grid = std::min(args.n_items, sm_count());
   const int smem_k = rs_smem_bytes(args.k16);
-  static int a_tmem = -1;      // B200TIP_A_TMEM=0|1: A operand of the resident kernel from tensor memory
-  if (a_tmem < 0) {
-    const char* e = getenv("B200TIP_A_TMEM");
-    a_tmem = e ? (e[0] == '1' ? 1 : 0) : kATmemDefault;
-  }
-  args.a_tmem = a_tmem;
 #define TIP_RS_CASE(K)                                                                                   \
   case K:                                                                                                \
     pair_rs_kernel<MODE, K, EXCL><<<grid, kRsThreads, smem_k, st>>>(ma, mat, mb, mbt, args);               \
@@ -1477,17 +1148,6 @@ static int launch_pair_rs(const void* q_pack, int64_t m, const void* t_pack, int
 #undef TIP_RS_CASE
   TIP_LAUNCH_CHECK();
   return TIP_OK;
-}
-
-// The CTA-pair streaming kernel serves long traces when B200TIP_PAIR2=1 (default set by kPair2Default)
-constexpr int kPair2Default = 0;
-static bool use_pair2() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("B200TIP_PAIR2");
-    v = e ? (e[0] == '1' ? 1 : 0) : kPair2Default;
-  }
-  return v == 1;
 }
 
 static int k16_of(int64_t d, int segments) {
@@ -1544,9 +1204,6 @@ extern "C" int tip_nn_filter(const void* q_pack, const float* q_sqnorm, int64_t 
   if (a.k16 <= kRsMaxK16)
     return excl ? launch_pair_rs<MODE_NN, true>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream)
                 : launch_pair_rs<MODE_NN, false>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
-  if (use_pair2())
-    return excl ? launch_pair2<MODE_NN, true>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream)
-                : launch_pair2<MODE_NN, false>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
   return excl ? launch_pair<MODE_NN, true>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream)
               : launch_pair<MODE_NN, false>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
 }
@@ -1554,19 +1211,18 @@ extern "C" int tip_nn_filter(const void* q_pack, const float* q_sqnorm, int64_t 
 extern "C" int tip_nn_filter_tile(int64_t d, int32_t* q_rows, int32_t* t_rows) {
   TIP_REQUIRE(d >= 1 && q_rows && t_rows, "arguments");
   const bool rs = k16_of(d, 1) <= kRsMaxK16;
-  *q_rows = rs ? RS_BM : (use_pair2() ? 2 * BM : BM);
+  *q_rows = rs ? RS_BM : BM;
   *t_rows = rs ? RS_BN : BN;
   return TIP_OK;
 }
 
 extern "C" int tip_nn_filter_kind(int64_t d) {
   if (d < 1) return -1;
-  if (k16_of(d, 1) <= kRsMaxK16) return 1;
-  return use_pair2() ? 2 : 0;
+  return k16_of(d, 1) <= kRsMaxK16 ? 1 : 0;
 }
 
-extern "C" int tip_kde_tile_rows(void) { return use_pair2() ? 2 * BM : BM; }
-extern "C" int tip_kde_slot_parts(void) { return use_pair2() ? 2 : kLseEpiWarps / 4; }
+extern "C" int tip_kde_tile_rows(void) { return BM; }
+extern "C" int tip_kde_slot_parts(void) { return kLseEpiWarps / 4; }
 
 extern "C" int tip_kde_lse(const void* q_pack, int64_t m, const void* t_pack, int64_t n, int64_t d, int64_t pitch,
                            const tip_work_item* items, int32_t n_items, float* part_max, float* part_sum,
@@ -1577,7 +1233,6 @@ extern "C" int tip_kde_lse(const void* q_pack, int64_t m, const void* t_pack, in
   PairArgs a{};
   a.items = items; a.n_items = n_items; a.n_static = n_items; a.k16 = k16_of(d, 3); a.m = m;
   a.part_max = part_max; a.part_sum = part_sum;
-  if (use_pair2()) return launch_pair2<MODE_LSE>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
   return launch_pair<MODE_LSE>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
 }
 
@@ -1590,10 +1245,6 @@ extern "C" int tip_kde_lse_f16(const void* q_pack, int64_t m, const void* t_pack
   PairArgs a{};
   a.items = items; a.n_items = n_items; a.n_static = n_items; a.k16 = k16_of(d, 1); a.m = m;
   a.part_max = part_max; a.part_sum = part_sum;
-  if (use_pair2()) {
-    a.idesc = kIdescP2F16;
-    return launch_pair2<MODE_LSE>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
-  }
   a.idesc = kIdescF16;
   return launch_pair<MODE_LSE>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
 }
@@ -1602,17 +1253,15 @@ extern "C" int tip_pair_probe(const void* q_pack, int64_t m, const void* t_pack,
                               int64_t pitch, int variant, float* out, void* stream) {
   TIP_REQUIRE(q_pack && t_pack && out, "null pointer");
   TIP_REQUIRE(pitch == tip_pair_pitch(d, segments), "pitch does not match tip_pair_pitch");
-  TIP_REQUIRE(variant >= 0 && variant <= 3, "variant: 0 auto, 1 streaming, 2 resident, 3 streaming CTA pair");
+  TIP_REQUIRE(variant >= 0 && variant <= 2, "variant: 0 auto, 1 streaming, 2 resident");
   static tip_work_item* d_item = nullptr;
   if (!d_item) TIP_CHECK_CUDA(cudaMalloc(&d_item, sizeof(tip_work_item)));
   const int k16 = k16_of(d, segments);
   const bool rs = variant == 2 || (variant == 0 && k16 <= kRsMaxK16);
-  const bool p2 = variant == 3 || (variant == 0 && !rs && use_pair2());
-  tip_work_item h{0, (int32_t)std::min<int64_t>(m, (rs || p2) ? RS_BM : BM), 0, (int32_t)std::min<int64_t>(n, 256), 0, 0};
+  tip_work_item h{0, (int32_t)std::min<int64_t>(m, rs ? RS_BM : BM), 0, (int32_t)std::min<int64_t>(n, 256), 0, 0};
   TIP_CHECK_CUDA(cudaMemcpyAsync(d_item, &h, sizeof(h), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   PairArgs a{};
   a.items = d_item; a.n_items = 1; a.n_static = 1; a.k16 = k16; a.m = m; a.dump = out;
   if (rs) return launch_pair_rs<MODE_DUMP>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
-  if (p2) return launch_pair2<MODE_DUMP>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
   return launch_pair<MODE_DUMP>(q_pack, m, t_pack, n, pitch, a, (cudaStream_t)stream);
 }

@@ -17,7 +17,6 @@
 // Both also emit the winner's original index and (optionally) copy the winning train row, which
 // is the query of DSA's second stage (surprise.py:627-629, 648).
 #include <algorithm>
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <vector>
@@ -101,10 +100,9 @@ __device__ __forceinline__ const T* query_row(const RerankArgs<T>& a, int64_t ro
   return a.q + (a.q_idx ? (int64_t)a.q_idx[row] : row) * (int64_t)a.d;
 }
 
-template <typename T, int NL = 32>
-__device__ __forceinline__ void write_result(const RerankArgs<T>& a, int64_t row, const Best<T>& b, int lane, int nlanes,
-                                             unsigned mask = 0xffffffffu) {
-  // all `nlanes` (== NL) threads of the caller hold the same `b`; `lane` in [0, NL)
+template <typename T>
+__device__ __forceinline__ void write_result(const RerankArgs<T>& a, int64_t row, const Best<T>& b, int lane) {
+  // all 32 lanes of the calling warp hold the same `b`
   if (lane == 0) {
     const T dist = b.pos >= 0 ? b.dist : (T)NAN;   // empty range -> NaN / -1
     a.out_dist[row] = dist;
@@ -124,13 +122,13 @@ __device__ __forceinline__ void write_result(const RerankArgs<T>& a, int64_t row
   const T* src = a.t + (int64_t)(b.pos < 0 ? 0 : b.pos) * a.d;
   if (a.out_rows) {
     T* dst = a.out_rows + row * (int64_t)a.d;
-    for (int i = lane; i < a.d; i += nlanes) dst[i] = b.pos >= 0 ? src[i] : (T)0;
+    for (int i = lane; i < a.d; i += 32) dst[i] = b.pos >= 0 ? src[i] : (T)0;
   }
   if (a.next_pack)
-    warp_pack_query<T, NL>(b.pos >= 0 ? src : nullptr, a.d, a.next_center, a.next_pack + row * a.next_pitch, a.next_pitch,
-                           a.next_sqnorm + row, a.next_rounderr ? a.next_rounderr + row : nullptr, a.next_row_min + row,
-                           a.next_cand_cnt + row, lane,
-                           (a.seed.ub && b.pos >= 0) ? a.seed.ub[b.pos] : __int_as_float(0x7f800000), &a.seed, mask);
+    warp_pack_query<T>(b.pos >= 0 ? src : nullptr, a.d, a.next_center, a.next_pack + row * a.next_pitch, a.next_pitch,
+                       a.next_sqnorm + row, a.next_rounderr ? a.next_rounderr + row : nullptr, a.next_row_min + row,
+                       a.next_cand_cnt + row, lane,
+                       (a.seed.ub && b.pos >= 0) ? a.seed.ub[b.pos] : __int_as_float(0x7f800000), &a.seed);
 }
 
 // ---- kernel 1: one warp per query, candidate lists ----------------------------------------------
@@ -169,7 +167,7 @@ rerank_list_kernel(const RerankArgs<T> a) {
   }
   if (cls < 0 || cls >= a.n_classes) {   // never scored by the reference either
     Best<T> none{Rn<T>::inf(), 0x7fffffff, -1};
-    write_result(a, row, none, lane, 32);
+    write_result(a, row, none, lane);
     return;
   }
   if (a.cand_cnt == nullptr || cnt < 1 || cnt > a.cap) {
@@ -250,95 +248,7 @@ rerank_list_kernel(const RerankArgs<T> a) {
   }
   // (no global statistics here: one same-address atomic per query serialises in L2; candidate
   // counts can be read from cand_cnt)
-  write_result(a, row, best, lane, 32);
-}
-
-// ---- kernel 1b: one 8-lane GROUP per query (short traces) ---------------------------------------------
-// A query's candidate list is ~3 rows, so a whole warp per query leaves three of its four 8-lane groups idle
-// and the kernel is a chain of dependent memory latencies with too few queries in flight: 10 000 queries are
-// 2.1 waves of resident warps.  Here every group owns a query (4 per warp): the same per-row arithmetic
-// (NumPy's leaf: the lane's stride-8 accumulator, tree by xor-shuffles inside the group), entries walked
-// sequentially by the group, everything resident in one wave.
-template <typename T>
-__global__ void __launch_bounds__(256, sizeof(T) == 4 ? 4 : 1) rerank_group_kernel(const RerankArgs<T> a) {
-  using R = Rn<T>;
-  const int lane = threadIdx.x & 31;
-  const int sub = lane & 7, grp = lane >> 3;
-  const int64_t row = ((int64_t)blockIdx.x * 8 + (threadIdx.x >> 5)) * 4 + grp;
-  if (row >= a.m) return;                       // uniform inside a group; groups only ever sync among themselves
-  const unsigned gmask = 0xFFu << (lane & 24);
-  const int cnt = a.cand_cnt ? a.cand_cnt[row] : 0;
-  const int cls = a.q_class ? a.q_class[row] : 0;
-  const bool spec = a.cand_cnt != nullptr;
-  int2 first = make_int2(0, 0);
-  if (spec) first = *reinterpret_cast<const int2*>(a.cand_idx + row * (int64_t)a.cap * 2);
-  const T* x = query_row(a, row);
-  const int n = a.d;
-  const int lim = n - (n % 8);
-  T xr[16], xt[7];
-#pragma unroll
-  for (int u = 0; u < 16; u++) xr[u] = 8 * u + sub < lim ? x[8 * u + sub] : (T)0;
-#pragma unroll
-  for (int u = 0; u < 7; u++) xt[u] = lim + u < n ? x[lim + u] : (T)0;
-  if (cls < 0 || cls >= a.n_classes) {   // never scored by the reference either
-    Best<T> none{Rn<T>::inf(), 0x7fffffff, -1};
-    write_result<T, 8>(a, row, none, sub, 8, gmask);
-    return;
-  }
-  if (a.cand_cnt == nullptr || cnt < 1 || cnt > a.cap) {
-    if (sub == 0) {
-      if (a.count_only) atomicAdd(a.work, 1);
-      else a.work[1 + atomicAdd(a.work, 1)] = (int32_t)row;
-    }
-    return;
-  }
-  const int c0 = a.class_off[cls], c1 = a.class_off[cls + 1], cn = a.class_off[a.n_classes];
-  Best<T> best{Rn<T>::inf(), 0x7fffffff, -1};
-  for (int e = 0; e < cnt; e++) {
-    int2 ent = first;
-    if (e > 0) ent = *reinterpret_cast<const int2*>(a.cand_idx + (row * (int64_t)a.cap + e) * 2);
-    const int start = ent.x;
-    unsigned cmask = (unsigned)ent.y;
-    while (cmask) {
-      const int bit = __ffs(cmask) - 1;
-      cmask &= cmask - 1;
-      const int j = start + bit;
-      if (j < 0 || j >= a.n) continue;
-      const int gid = a.t_gid ? a.t_gid[j] : j;
-      const T* y = a.t + (int64_t)j * a.d;
-      T yr[16], yt[7];
-#pragma unroll
-      for (int u = 0; u < 16; u++) yr[u] = 8 * u + sub < lim ? y[8 * u + sub] : (T)0;
-#pragma unroll
-      for (int u = 0; u < 7; u++) yt[u] = lim + u < n ? y[lim + u] : (T)0;
-      T r = (T)0;
-      if (lim > 0) {
-        T d0 = R::sub(xr[0], yr[0]);
-        r = R::mul(d0, d0);
-#pragma unroll
-        for (int u = 1; u < 16; u++) {
-          if (8 * u < lim) {
-            const T du = R::sub(xr[u], yr[u]);
-            r = R::add(r, R::mul(du, du));
-          }
-        }
-        r = R::add(r, __shfl_xor_sync(gmask, r, 1));
-        r = R::add(r, __shfl_xor_sync(gmask, r, 2));
-        r = R::add(r, __shfl_xor_sync(gmask, r, 4));
-      }
-#pragma unroll
-      for (int u = 0; u < 7; u++) {
-        if (lim + u < n) {
-          const T du = R::sub(xt[u], yt[u]);
-          r = R::add(r, R::mul(du, du));
-        }
-      }
-      const bool in_range = a.mode == TIP_RANGE_SAME_CLASS ? (j >= c0 && j < c1) : (j < cn && (j < c0 || j >= c1));
-      if (in_range) consider(best, Rn<T>::sqrt(r), gid, j);   // all 8 lanes agree
-    }
-  }
-  __syncwarp(gmask);
-  write_result<T, 8>(a, row, best, sub, 8, gmask);
+  write_result(a, row, best, lane);
 }
 
 // ---- kernels 2+3: exhaustive scan of the class range for queued queries ---------------------------
@@ -393,7 +303,7 @@ __device__ __forceinline__ void rerank_merge(const RerankArgs<T>& a, int queued)
       best = merge(best, od, og, op);
     }
     if (lane == 0 && a.stats) atomicAdd(a.stats + 0, 1ULL);
-    write_result(a, a.work[1 + w], best, lane, 32);
+    write_result(a, a.work[1 + w], best, lane);
   }
 }
 
@@ -457,37 +367,11 @@ __global__ void __launch_bounds__(kScanThreads) rerank_scan_kernel(const RerankA
 template <typename T>
 static int launch_rerank(const RerankArgs<T>& a, cudaStream_t st) {
   // precondition (and postcondition): work[0] == 0 and work[1 + m] == 0
-  // B200TIP_RERANK_GROUPS=1: one 8-lane group per query (measured SLOWER at C2: 0.216 vs 0.199 ms per step — four
-  // divergent queries per warp serialise more than the extra resident queries buy); default: one warp per query
-  static int group_mode = -1;
-  if (group_mode < 0) {
-    const char* e = getenv("B200TIP_RERANK_GROUPS");
-    group_mode = (e && e[0] == '1') ? 1 : 0;
-  }
-  static bool pref_scan = false;
-  prefer_max_shared(rerank_scan_kernel<T>, &pref_scan);
-  static int wpb = 0;      // B200TIP_RERANK_WPB = 1 | 2 | 8 queries per block (bring-up A/B)
-  if (wpb == 0) {
-    const char* e = getenv("B200TIP_RERANK_WPB");
-    wpb = (e && (atoi(e) == 1 || atoi(e) == 2 || atoi(e) == 8)) ? atoi(e) : -1;
-  }
-  // measured at C2 (one box, ms per step): 8 -> 0.1943, 2 -> 0.1926, 1 -> 0.1928; long traces (C5 slice): 40.4 / 40.6 / 40.9
-  const int w = wpb > 0 ? wpb : (a.d <= 128 ? 2 : 8);
-  const unsigned nb = (unsigned)((a.m + w - 1) / w);
-  if (a.d <= 128 && group_mode) rerank_group_kernel<T><<<(unsigned)((a.m + 31) / 32), 256, 0, st>>>(a);
-  else if (a.d == 128) {
-    if (w == 1) rerank_list_kernel<T, true, 1, true><<<nb, 32, 0, st>>>(a);
-    else if (w == 2) rerank_list_kernel<T, true, 2, true><<<nb, 64, 0, st>>>(a);
-    else rerank_list_kernel<T, true, 8, true><<<nb, 256, 0, st>>>(a);
-  } else if (a.d <= 128) {
-    if (w == 1) rerank_list_kernel<T, true, 1><<<nb, 32, 0, st>>>(a);
-    else if (w == 2) rerank_list_kernel<T, true, 2><<<nb, 64, 0, st>>>(a);
-    else rerank_list_kernel<T, true, 8><<<nb, 256, 0, st>>>(a);
-  } else {
-    if (w == 1) rerank_list_kernel<T, false, 1><<<nb, 32, 0, st>>>(a);
-    else if (w == 2) rerank_list_kernel<T, false, 2><<<nb, 64, 0, st>>>(a);
-    else rerank_list_kernel<T, false, 8><<<nb, 256, 0, st>>>(a);
-  }
+  // queries (warps) per block, measured with 8 / 2 / 1 (one box): C2 0.1943 / 0.1926 / 0.1928 ms per step, long traces
+  // (C5 slice) 40.4 / 40.6 / 40.9.  One 8-lane group per query instead of a warp was slower at C2 (0.216 vs 0.199 ms).
+  if (a.d == 128) rerank_list_kernel<T, true, 2, true><<<(unsigned)((a.m + 1) / 2), 64, 0, st>>>(a);
+  else if (a.d < 128) rerank_list_kernel<T, true, 2><<<(unsigned)((a.m + 1) / 2), 64, 0, st>>>(a);
+  else rerank_list_kernel<T, false, 8><<<(unsigned)((a.m + 7) / 8), 256, 0, st>>>(a);
   TIP_LAUNCH_CHECK();
   if (a.count_only) return TIP_OK;   // speculative call: no exhaustive-scan launch, the caller inspects work[0]
   // normally an empty queue: every block returns at once, so keep the grid small (the fallback itself is rare)

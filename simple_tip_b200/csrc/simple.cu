@@ -25,15 +25,6 @@ void set_error(const char* fmt, ...) {
 }
 void count_launch(int n) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); }
 
-bool carveout_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("B200TIP_CARVEOUT");
-    on = (e && e[0] == '1') ? 1 : 0;
-  }
-  return on == 1;
-}
-
 int sm_count() {
   static int cached = 0;
   if (!cached) {
@@ -856,17 +847,12 @@ extern "C" int tip_kmnc(const void* act, int act_dtype, int64_t n, int64_t d, co
                                            : (const void*)kmnc_strip_kernel<int32_t, true>;
         const int which = bucket == nullptr ? 0 : (i16 ? 1 : 2);
         static int per_sm_of[3] = {0, 0, 0};   // occupancy of each instance (same on every device of a box)
-        static int waves = 0;                   // B200TIP_KMNC_WAVES: grid in resident waves (bring-up knob, default 1)
         if (per_sm_of[which] == 0) {
           int v = 0;
           TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, fn, 256, 0));
           per_sm_of[which] = std::max(v, 1);
         }
-        if (waves == 0) {
-          const char* e = getenv("B200TIP_KMNC_WAVES");
-          waves = (e && atoi(e) >= 1 && atoi(e) <= 64) ? atoi(e) : 1;
-        }
-        const int64_t resident = (int64_t)sm_count() * per_sm_of[which] * waves;
+        const int64_t resident = (int64_t)sm_count() * per_sm_of[which];
         const int64_t lanes = std::max<int64_t>(1, std::min<int64_t>(resident / nstrips, n / (2 * kStripRows)));
         const int ns = (int)nstrips, ln = (int)lanes;
         const float* a = (const float*)act;
@@ -918,8 +904,6 @@ static int pair_prep_impl(const void* src, int dtype, int64_t rows, int64_t d, c
   const int64_t blocks = (rows + 7) / 8;
   TIP_REQUIRE(blocks < (1LL << 31), "too many rows");
   cudaStream_t st = (cudaStream_t)stream;
-  static bool pref_f = false;
-  prefer_max_shared(pair_prep_kernel<float>, &pref_f);
   if (dtype == TIP_F32)
     pair_prep_kernel<float><<<(unsigned)blocks, 256, 0, st>>>((const float*)src, rows, (int)d, center, role, segments,
                                                              scale, norm_coef, (__nv_bfloat16*)dst, pitch, sqnorm,

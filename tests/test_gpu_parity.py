@@ -31,12 +31,10 @@ def _torch():
 # ------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("d,segments,variant", [(16, 1, 1), (16, 1, 2), (128, 1, 1), (128, 1, 2), (100, 1, 0),
                                                 (64, 1, 2), (120, 1, 2), (5, 1, 2), (300, 1, 0), (2048, 1, 0),
-                                                (10, 3, 0), (256, 3, 0), (40, 3, 1), (40, 3, 2),
-                                                (16, 1, 3), (300, 1, 3), (2048, 1, 3), (256, 3, 3)])
+                                                (10, 3, 0), (256, 3, 0), (40, 3, 1), (40, 3, 2)])
 def test_pair_probe_matches_packed_matmul(d, segments, variant):
     """variant 1 = streaming kernel (128 x 256 tiles), 2 = resident-query kernel (256 x 192 tiles,
-    128-byte-swizzled chunks + 32-byte-swizzled tail panels), 3 = streaming CTA-pair kernel (cta_group::2,
-    256 x 256 tiles), 0 = whatever tip_nn_filter picks."""
+    128-byte-swizzled chunks + 32-byte-swizzled tail panels), 0 = whatever tip_nn_filter picks."""
     torch = _torch()
     from simple_tip_b200 import _lib
     from simple_tip_b200 import engine as E
@@ -52,9 +50,7 @@ def test_pair_probe_matches_packed_matmul(d, segments, variant):
     if variant == 2 and k16 > 9:
         pytest.skip("packed row too wide for the resident-query kernel")
     resident = variant == 2 or (variant == 0 and k16 <= 9)
-    pair2 = variant == 3 or (variant == 0 and not resident and int(lib.tip_nn_filter_kind(d)) == 2 and segments == 1) \
-        or (variant == 0 and not resident and int(lib.tip_kde_tile_rows()) == 256)
-    rows = 256 if (resident or pair2) else 128
+    rows = 256 if resident else 128
     qp = torch.empty((256, pitch), dtype=torch.bfloat16, device=dev)
     tp = torch.empty((256, pitch), dtype=torch.bfloat16, device=dev)
     qs = torch.empty(256, dtype=torch.float32, device=dev)
